@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — tokens/s + acceptance rate of self-speculative decoding (BASELINE.json metric).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 A STEP is one full generation: a 128-id synthetic prompt -> a 512-token greedy continuation,
 Llama-2-7B architecture, random-init weights (seeded), exit_layer 8, num_speculations 6 —
@@ -16,6 +16,9 @@ times it (self_speculation/generator_base.py:107-129).
   N > 1  : one process per GPU (torchrun).  The path is batch-1 decoding, so ranks are
            independent replicas serving different prompts (weak scaling, no data-path
            collective); `--tp` instead shards ONE model tensor-parallel over the N GPUs.
+  --dump-outputs DIR : after the timed steps, what the last timed generation returned (tokens,
+           acceptance, per-round results) as DIR/<name>.npy.  Weights and prompts are seeded, so
+           runs with the same arguments see the same inputs and two builds compare output for output.
 
 `--impl reference` times the reference algorithm's CPU implementation (the oracle port of
 /root/reference/self_speculation/*, which cannot travel to the GPU box) on the host cores, on a
@@ -61,7 +64,14 @@ def parse_args():
     ap.add_argument("--cpu-max-steps", type=int, default=0, help="reference arm: tokens per step")
     ap.add_argument("--cpu-budget", type=float, default=300.0,
                     help="reference arm: seconds of CPU time the K timed generations may take in total")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed generation returned as DIR/<name>.npy (rank 0)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the engine arm (--impl b200)")
+    return args
 
 
 # --------------------------------------------------------------------------------------------
@@ -357,19 +367,20 @@ class Watchdog:
 def measure_generations(strat, eng, model, prompts, gcfg, args, eos, first, count, e2e=False):
     """`count` generations starting at prompt index `first`, device-timed: CUDA events on the
     engine's stream around prefill and every round, inputs already resident."""
-    out = dict(tokens=0, dev_ms=0.0, bytes=0.0, accs=[], streams=[])
+    out = dict(tokens=0, dev_ms=0.0, bytes=0.0, accs=[], streams=[], last_rounds=[])
     for i in range(count):
         prompt = prompts[(first + i) % len(prompts)]
         eng.begin(exit_layer=gcfg.exit_layer, max_steps=gcfg.max_steps, eos_token_ids=eos)
         eng.prefill(prompt)
         ms = eng.last_device_ms
-        toks, matches, drafted = [], 0, 0
+        toks, matches, drafted, rounds = [], 0, 0, []
         while len(toks) < gcfg.max_steps:
             d = min(gcfg.num_speculations, gcfg.max_steps - len(toks) - 1)
             ctx = eng.kv_len
             r = eng.round(d)
             ms += eng.last_device_ms
             out["bytes"] += eng.round_bytes(d, ctx)
+            rounds.append(r)
             toks += r.emitted
             matches += r.n_matches
             drafted += r.n_drafted
@@ -380,7 +391,29 @@ def measure_generations(strat, eng, model, prompts, gcfg, args, eos, first, coun
         out["dev_ms"] += ms
         out["accs"].append(matches / max(1, drafted))
         out["streams"].append(toks)
+        out["last_rounds"] = rounds
     return out
+
+
+def dump_outputs(out_dir, meas):
+    """What the timed path handed its caller in the last timed generation, as float64 .npy
+    (token ids are exact below 2^53): the generated tokens, the generation's acceptance rate and
+    every round's lsk_round_out fields; ragged per-round id lists are concatenated in round order."""
+    import numpy as np
+    rounds = meas["last_rounds"]
+    arrays = {
+        "tokens": meas["streams"][-1],
+        "acceptance_rate": [meas["accs"][-1]],
+        "round_n_drafted": [r.n_drafted for r in rounds],
+        "round_n_matches": [r.n_matches for r in rounds],
+        "round_kv_len": [r.kv_len for r in rounds],
+        "round_draft_ids": [t for r in rounds for t in r.draft],
+        "round_verified_ids": [t for r in rounds for t in r.verified],
+        "round_emitted_ids": [t for r in rounds for t in r.emitted],
+    }
+    os.makedirs(out_dir, exist_ok=True)
+    for name, values in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.asarray(values, dtype=np.float64))
 
 
 def class_profile(eng, arch, tp, prompts, gcfg, eos, reps=5):
@@ -653,6 +686,8 @@ def run_b200_arm(args):
     meas = measure_generations(strat, eng, model, my_prompts, gcfg, args, eos, args.warmup, args.steps, e2e=False)
     barrier()
     launches = eng.launch_count - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, meas)
     # e2e leg through the plug-in call (wall clock, host ids in / host ids out, every copy and the
     # per-round sync inside the region)
     e2e = dict(tokens_e2e=0, wall=0.0, rounds=0)

@@ -227,5 +227,27 @@ def main() -> None:
     print("wrote", GOLDEN_DIR)
 
 
+RERUN_CASE = "mha128_a0.1"
+
+
+def rerun() -> None:
+    """Run the reference once more on one committed case (seeded weights, prompt, eos and settings
+    read back from spec_traces.json) and store its whole result as reference_rerun.json, so the
+    suite can check the fixture against an independent run without the reference tree."""
+    import transformers
+    ref = ref_shim.load_reference()
+    with open(os.path.join(GOLDEN_DIR, "spec_traces.json")) as f:
+        case = next(c for c in json.load(f)["cases"] if c["name"] == RERUN_CASE)
+    dims = orc.LlamaDims(*case["dims"])
+    sd = orc.random_state_dict(dims, case["weight_seed"], case["damp_from"], case["alpha"])
+    res = run_reference(ref, build_hf(dims, sd), case["prompt"], case["eos"], case["cfg"],
+                        case.get("torch_seed"))
+    with open(os.path.join(GOLDEN_DIR, "reference_rerun.json"), "w") as f:
+        json.dump(dict(generator="oracle/gen_golden.py --rerun", case=RERUN_CASE,
+                       torch=torch.__version__, transformers=transformers.__version__,
+                       reference=res), f, indent=1)
+    print("wrote", os.path.join(GOLDEN_DIR, "reference_rerun.json"))
+
+
 if __name__ == "__main__":
-    main()
+    rerun() if "--rerun" in sys.argv else main()

@@ -3,8 +3,7 @@
 Lets `/root/reference/self_speculation/*.py` (written against transformers ~4.45, pinned
 4.50.0 in `/root/reference/requirements.txt:4`) import and run under the transformers 5.5
 installed in this image, WITHOUT editing or copying any reference file.  Used only by
-`oracle/gen_golden.py` (to produce `tests/golden/*.json`) and by CPU tests that are skipped
-when `/root/reference` is absent (it does not exist on the GPU box).
+`oracle/gen_golden.py` (to produce `tests/golden/*.json`).
 
 What is patched at run time (SURVEY.md Appendix B):
   * `colorama` is not installed            -> stub module (only used for TTY colours,
