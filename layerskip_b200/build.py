@@ -15,10 +15,8 @@ PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG_DIR, "csrc")
 LIB_PATH = os.path.join(PKG_DIR, "liblsk.so")
 STAMP_PATH = os.path.join(PKG_DIR, ".liblsk.stamp")
+INCLUDE_DIR = os.path.join(os.path.dirname(PKG_DIR), "include")
 SOURCES = ["engine.cu"]
-HEADERS = ["common.cuh", "gemm_skinny.cuh", "attention.cuh", "misc_kernels.cuh", "sampling.cuh",
-           "tp_peer.cuh", "lmhead_tc.cuh",
-           os.path.join("..", "..", "include", "lsk.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
@@ -26,13 +24,20 @@ NVCC_FLAGS = [
 ]
 
 
+def _digest_inputs() -> list:
+    """Every file the library is compiled from: all of csrc/ (engine.cu includes the headers,
+    so a new header needs no list to be kept in step) and the public C header."""
+    files = [os.path.join(CSRC, n) for n in sorted(os.listdir(CSRC))]
+    files.append(os.path.join(INCLUDE_DIR, "lsk.h"))
+    return [p for p in files if os.path.isfile(p)]
+
+
 def _digest() -> str:
     h = hashlib.sha256()
-    for name in SOURCES + HEADERS:
-        path = os.path.join(CSRC, name)
-        if os.path.exists(path):
-            with open(path, "rb") as f:
-                h.update(f.read())
+    for path in _digest_inputs():
+        h.update(os.path.basename(path).encode() + b"\0")
+        with open(path, "rb") as f:
+            h.update(f.read())
     h.update(" ".join(NVCC_FLAGS).encode())
     return h.hexdigest()
 

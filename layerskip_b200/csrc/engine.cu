@@ -147,7 +147,8 @@ struct lsk_engine {
   float* rank_val = nullptr;           // TP: [16]
   int* rank_idx = nullptr;
   int* d_zero = nullptr;
-  int* d_prompt = nullptr;             // [max_ctx] prompt ids
+  int* d_prompt = nullptr;             // [max_ctx] prompt ids, then the emitted tokens (n-gram ban history)
+  int* d_dbg_ids = nullptr;            // [kMaxRows] ids of lsk_debug_forward_rows (kept out of the history)
   DevState* state = nullptr;
   GenParams* gen_dev = nullptr;
   RoundResult* res_host = nullptr;     // mapped pinned
@@ -155,7 +156,6 @@ struct lsk_engine {
 
   GemmPlan p_qkv, p_o, p_gu, p_d, p_lm;
   size_t l2_prefetch_bytes = 0;          // LSK_L2_PREFETCH_MB: head of the NEXT kernel's weights pulled into L2 (A/B: no gain, +11 % traffic -> off)
-  int lm_cand = 0;                     // candidates produced by the LM head (its grid)
   const float* cur_cand_val = nullptr;  // candidates of the last enqueued LM head (epilogue's, or the banned rows' arg-max)
   const int* cur_cand_idx = nullptr;
   int cur_n_cand = 0;
@@ -740,7 +740,10 @@ static int enqueue_lm_head(lsk_engine* e, int row0, int M, int j0, const void* a
   e->cur_class = CLS_MISC;
   const float* cv = e->cand_val;
   const int* ci = e->cand_idx;
-  int ncand = e->lm_cand;
+  // one candidate per CTA of the launch above.  The even-wave grid of the skinny GEMM can be
+  // smaller than min(tiles, SMs); a slot no CTA wrote would hold a stale (0.0, index 0) pair and
+  // win every row whose logits are all negative.
+  int ncand = e->lm_tc ? e->lm_tc_grid : plan_sched(M <= 8 ? 1 : 2, M, PRO_RMS, EPI_LMHEAD, e->p_lm, e->sm_count).grid;
   if (ban) {
     CU(launch(e, ngram_ban_kernel, dim3(M), dim3(256), 0, e->logits, e->vocab_l_pad, e->vocab_l, e->vocab_off,
               (const int*)e->d_prompt, (const DevState*)e->state, (int)e->gen.no_repeat_ngram_size, j0));
@@ -993,7 +996,6 @@ static int create_into(lsk_engine* e, const lsk_config& c) {
   e->p_gu = make_plan(2 * e->inter_l, c.hidden, e->sm_count);
   e->p_d = make_plan(c.hidden, e->inter_l_pad, e->sm_count);
   e->p_lm = make_plan(e->vocab_l_pad, c.hidden, e->sm_count);
-  e->lm_cand = e->p_lm.n_tiles < e->sm_count ? e->p_lm.n_tiles : e->sm_count;
   if (const char* env = getenv("LSK_L2_PREFETCH_MB")) e->l2_prefetch_bytes = (size_t)atoi(env) << 20;
   if (getenv("LSK_LMHEAD_TC") && atoi(getenv("LSK_LMHEAD_TC")) != 0) {
     // tcgen05 LM head: needs hidden % 64 == 0 and the 16-token B operand + a >= 3-stage ring in
@@ -1006,7 +1008,6 @@ static int create_into(lsk_engine* e, const lsk_config& c) {
       e->lm_tc_tiles = (e->vocab_l + kTcTileRows - 1) / kTcTileRows;
       const int waves = (e->lm_tc_tiles + e->sm_count - 1) / e->sm_count;
       e->lm_tc_grid = (e->lm_tc_tiles + waves - 1) / waves;        // even waves
-      e->lm_cand = e->lm_tc_grid;
     } else {
       fprintf(stderr, "[lsk] LSK_LMHEAD_TC ignored: hidden %d does not fit the tcgen05 LM head\n", c.hidden);
     }
@@ -1090,6 +1091,7 @@ static int create_into(lsk_engine* e, const lsk_config& c) {
   TRY(alloc((void**)&e->rank_idx, kMaxRows * 4));
   TRY(alloc((void**)&e->d_zero, 4));
   TRY(alloc((void**)&e->d_prompt, (size_t)e->max_pos * 4));
+  TRY(alloc((void**)&e->d_dbg_ids, kMaxRows * 4));
   TRY(alloc((void**)&e->state, sizeof(DevState)));
   TRY(alloc((void**)&e->gen_dev, sizeof(GenParams)));
   CU(cudaHostAlloc((void**)&e->res_host, sizeof(RoundResult), cudaHostAllocMapped));
@@ -1150,7 +1152,7 @@ void lsk_destroy(lsk_engine* e) {
   void* ptrs[] = {e->embed, e->final_norm, e->lm_head, e->lm_head_tc, e->kpool, e->vpool, e->page_table, e->rope,
                   e->hidden, e->qbuf, e->attn_out, e->act, e->tp_buf, e->logits, e->logits_gath, e->logits_full, e->probs_d, e->probs_v, e->samp_scratch, e->cand_val,
                   e->cand_idx, e->gath_val, e->gath_idx, e->ban_val, e->ban_idx, e->rank_val, e->rank_idx,
-                  e->d_zero, e->d_prompt, e->state, e->gen_dev};
+                  e->d_zero, e->d_prompt, e->d_dbg_ids, e->state, e->gen_dev};
   for (void* p : ptrs) if (p) cudaFree(p);
   if (e->res_host) cudaFreeHost(e->res_host);
   if (e->ev0) cudaEventDestroy(e->ev0);
@@ -1547,10 +1549,11 @@ int lsk_debug_forward_rows(lsk_engine* e, const int32_t* ids, int32_t m) {
   const lsk_config& c = e->cfg;
   for (int i = 0; i < m; ++i)
     if (ids[i] < 0 || ids[i] >= c.vocab) return fail(LSK_ERR_INVALID, "token id %d out of range", ids[i]);
-  CU(cudaMemcpyAsync(e->d_prompt, ids, (size_t)m * 4, cudaMemcpyHostToDevice, e->stream));
+  // staged in a buffer of their own: d_prompt is the token history the n-gram ban reads
+  CU(cudaMemcpyAsync(e->d_dbg_ids, ids, (size_t)m * 4, cudaMemcpyHostToDevice, e->stream));
   e->cur_class = CLS_MISC;
   CU(launch(e, embed_tokens_kernel, dim3(m), dim3(256), 0, (const __nv_bfloat16*)e->embed, c.hidden,
-            (const int*)e->d_prompt, e->hidden, c.hidden));
+            (const int*)e->d_dbg_ids, e->hidden, c.hidden));
   for (int l = 0; l < c.n_layers; ++l) TRY(enqueue_layer(e, l, 0, m, &e->state->len, 0));
   const int keep_sample = e->gen.sample;
   e->gen.sample = 0;

@@ -71,3 +71,36 @@ def test_engine_with_tcgen05_lm_head_stays_exact_and_within_the_margin_gate(name
         spec.engines.close()
     assert s.predicted_tokens == a.predicted_tokens
     assert flips <= 4, gaps
+
+
+@pytest.mark.parametrize("value", [0.5, -0.001], ids=["positive", "all_negative"])
+@pytest.mark.parametrize("n,i,j", [(1005, 5, 1002), (1005, 130, 1001), (32001, 37 * 16 + 11, 31999)])
+def test_tcgen05_lm_head_tie_goes_to_the_lowest_index_and_padding_rows_never_win(n, i, j, value):
+    """Rows i < j (different 128-row tiles and rows inside them) each hold `value` in one column and
+    zeros elsewhere; the normed activations are exactly 1, so both logits equal `value` bit for bit.
+    Every other row is negative everywhere.  With n % 16 != 0 the last tile has padding rows, which
+    would win with logit 0 when `value` < 0 if they leaked into the arg-max."""
+    import ctypes as C
+    from layerskip_b200 import _lib
+    lib = _lib.load()
+    k, m = 256, 7
+    g = torch.Generator(device="cuda").manual_seed(n + i)
+    w = -(torch.rand(n, k, generator=g, device="cuda") * 0.01 + 0.001)
+    w[i] = 0
+    w[j] = 0
+    w[i, 3] = value
+    w[j, k - 5] = value
+    w = w.to(torch.bfloat16)
+    x = torch.ones(m, k, device="cuda")
+    nw = torch.ones(k, dtype=torch.bfloat16, device="cuda")
+    logits = torch.full((m, n), float("nan"), device="cuda")
+    bv = torch.zeros(16, device="cuda")
+    bi = torch.zeros(16, dtype=torch.int32, device="cuda")
+    ms = C.c_float(0)
+    torch.cuda.synchronize()
+    _lib.check(lib.lsk_test_lmhead_tc(w.data_ptr(), n, k, x.data_ptr(), nw.data_ptr(), 1e-5, m,
+                                      logits.data_ptr(), bv.data_ptr(), bi.data_ptr(), 1, C.byref(ms)))
+    torch.cuda.synchronize()
+    assert torch.equal(logits[:, i], logits[:, j]) and torch.equal(logits[:, i], logits.max(-1).values)
+    assert bi[:m].tolist() == [i] * m
+    assert torch.equal(bv[:m], logits[:, i])
